@@ -245,16 +245,16 @@ def run_ours(args, rank, world, local_rank):
     nb = max(1, SAMPLES_PER_GPU // args.batch)                    # calibration batches per step (= per whole calibration)
     cal = ArenaCalibrator(T, device, bins=BINS, num_of_bits=8, method='kl')
     stream = torch.cuda.current_stream()
-    hist_events, mm_events, launches = [], [], [0]
+    hist_events, mm_events, launches, last_weights = [], [], [0], [None]
     wq = MultiWeightQuantizer(wl.w, wl.w_scale, wl.w_offset, channel_axis=0)
 
     def weights_pass():
         if args.per_tensor_weight_launches:
-            for w, s, o in zip(wl.w, wl.w_scale, wl.w_offset): ext.QuantizeTensor_LC(w, s, o, -128, 127, 0, 0)
+            out = [ext.QuantizeTensor_LC(w, s, o, -128, 127, 0, 0) for w, s, o in zip(wl.w, wl.w_scale, wl.w_offset)]
             launches[0] += len(wl.w)
-        else:
-            wq()                                                  # all weights, one launch
-            launches[0] += 1
+            return out
+        launches[0] += 1
+        return wq()                                               # all weights, one launch
 
     def calibrate(timed):
         """One step: a whole two-phase calibration of this GPU's 512-sample share."""
@@ -266,11 +266,12 @@ def run_ours(args, rank, world, local_rank):
             if timed: e1.record(stream); mm_events.append((e0, e1))
         cal.end_phase()
         for k in range(nb):                                     # phase 2
-            weights_pass()
+            wq_out = weights_pass()
             if timed: e0 = torch.cuda.Event(enable_timing=True); e1 = torch.cuda.Event(enable_timing=True); e0.record(stream)
             cal.observe(wl.sets[k % args.rotate])
             if timed: e1.record(stream); hist_events.append((e0, e1))
         cal.end_phase()
+        last_weights[0] = wq_out
         return cal.scale
 
     def barrier():
@@ -314,6 +315,8 @@ def run_ours(args, rank, world, local_rank):
         per_rank = [torch.zeros_like(mine) for _ in range(world)]
         dist.all_gather(per_rank, mine)
     assert torch.isfinite(scales).all() and (scales > 0).all()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, cal, last_weights[0])
 
     # ---- roofline of the dominant kernel (multi-tensor histogram; 4 B/element) from the events of the timed region
     peak, peak_src = measured_peaks()
@@ -366,6 +369,24 @@ def run_ours(args, rank, world, local_rank):
     if rank == 0:
         result['cpu_baseline'] = cpu_baseline(args) if not args.no_cpu_baseline else None
     return result
+
+
+DUMP_WEIGHT_SAMPLE = 1 << 20
+
+
+def dump_outputs(out_dir, cal, weights):
+    """What the last timed step handed its caller, as .npy (float32, or float64 for the int32 histogram counts): the calibrated scales and
+    offsets with the statistics they came from (min/max, histogram scale, histogram arena), and a fixed sample (seed 0) of
+    DUMP_WEIGHT_SAMPLE elements of the fake-quantised weights, whose ~100 MB in full would not fit the 64 MB the dump may take."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    flat = torch.cat([w.reshape(-1) for w in weights])
+    idx = np.sort(np.random.RandomState(0).choice(flat.numel(), size=min(DUMP_WEIGHT_SAMPLE, flat.numel()), replace=False))
+    arrays = {'scale': cal.scale.float(), 'offset': cal.offset.float(), 'minmax': cal.minmax, 'hist_scale': cal.hist_scale,
+              'histogram': cal.hist.double(), 'weights_fakequant_sample': flat[torch.from_numpy(idx).to(flat.device)],
+              'weights_fakequant_sample_index': torch.from_numpy(idx.astype(np.float64))}
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + '.npy'), t.detach().cpu().numpy())
 
 
 def fakequant_sweep(ext, device, peak):
@@ -602,6 +623,8 @@ def main():
     ap.add_argument('--no-cpu-baseline', action='store_true', help='profiling runs only')
     ap.add_argument('--ref-budget', type=float, default=100.0, help='wall-clock budget (s) of the CPU reference arm')
     ap.add_argument('--per-tensor-weight-launches', action='store_true', help='one QuantizeTensor_LC launch per weight (the reference flow) instead of the multi-tensor launch')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write what the last one computed to DIR/<name>.npy (same arguments, same inputs: comparable across builds)')
     args = ap.parse_args()
     if args.batch is None: args.batch = WORKLOADS[args.workload]['batch']
     rank = int(os.environ.get('RANK', 0)); world = int(os.environ.get('WORLD_SIZE', 1)); local_rank = int(os.environ.get('LOCAL_RANK', 0))

@@ -23,6 +23,15 @@ def cases_of(npz, key='cases'):
     return json.loads(bytes(npz[key]).decode())
 
 
+def golden_input(npz, case):
+    """Input `x<k>` of a golden case: stored, or -- for uniform [0, 32) inputs -- regenerated from the seed and shape the case records
+    (tests/golden/make_golden.py draws them first from that seed)."""
+    k = case['k']
+    if f'x{k}' in npz.files:
+        return npz[f'x{k}']
+    return (np.random.RandomState(case['seed']).rand(*case['shape']) * 32).astype(np.float32)
+
+
 def seeded_batches(seed, n, shape, relu):
     """Same generator as tests/golden/make_golden.py::batches (numpy legacy RandomState: bit-stable)."""
     r = np.random.RandomState(seed)

@@ -141,8 +141,8 @@ def gen_linear_c():
             activate(cfg, s, o)
             y = PPQLinearQuantFunction(torch.from_numpy(x), cfg).numpy()
             q = PPQLinearQuant_toInt(torch.from_numpy(x), cfg).numpy()
-            out[f'x{k}'], out[f'y{k}'], out[f'q{k}'], out[f's{k}'], out[f'o{k}'] = x, y, q.astype(np.int32), s, o
-            cases.append(dict(k=k, axis=axis, qmin=0, qmax=255, mode=0))
+            out[f'y{k}'], out[f'q{k}'], out[f's{k}'], out[f'o{k}'] = y, q.astype(np.int32), s, o      # x: regenerated from seed + shape
+            cases.append(dict(k=k, axis=axis, qmin=0, qmax=255, mode=0, seed=3000 + k, shape=list(shape)))
             k += 1
     # signed weights, scales from the reference's per-channel minmax observer (BASELINE config 3 style)
     for shape in ([32, 3, 3, 3], [32, 1, 3, 3], [16, 32, 1, 1], [96, 1, 3, 3], [10, 64]):

@@ -1,8 +1,8 @@
 """Graph-level golden fixture: the UNMODIFIED reference pipeline (TRT_INT8 quantizer -> QuantizeFusionPass -> QuantizeSimplifyPass ->
 ParameterQuantizePass -> RuntimeCalibrationPass -> QuantAlignmentPass -> PassiveParameterQuantizePass -> ParameterBakingPass; CPU /
-torch path, USING_CUDA_KERNEL = False) run on a programmatically built BaseGraph (SURVEY.md appendix C2) in the build container.
+torch path, USING_CUDA_KERNEL = False) run on a programmatically built BaseGraph (SURVEY.md appendix C2).
 
-    python tests/golden/make_graph_golden.py          # rewrites tests/golden/graph_pipeline.npz
+    PPQ_REFERENCE_ROOT=<checkout> python tests/golden/make_graph_golden.py          # rewrites tests/golden/graph_pipeline.npz
 
 Stored: for every activation algorithm (kl, minmax, percentile, mse) every TensorQuantizationConfig's state / dominator / scale /
 offset right after RuntimeCalibrationPass and after the last pass, the quantised graph's output on the first batch, and the baked
@@ -56,7 +56,7 @@ def generate(ppq, net, methods):
 
 def main():
     ppq = refppq.load()
-    assert ppq is not None and refppq.root() == '/root/reference', 'generate fixtures from the read-only reference checkout'
+    assert ppq is not None and refppq.root() == os.environ.get('PPQ_REFERENCE_ROOT'), 'generate fixtures from a checkout named by $PPQ_REFERENCE_ROOT'
     from ppq.core import PPQ_CONFIG
     assert PPQ_CONFIG.USING_CUDA_KERNEL is False
     torch.set_num_threads(1)                                   # deterministic reductions

@@ -1,19 +1,17 @@
-"""Import the REAL reference package (OpenPPL/ppq) for tests -- test infrastructure only.
+"""Import the ORIGINAL PROJECT's package (OpenPPL/ppq, unmodified) -- test infrastructure, used only to record the golden results under
+tests/golden/ that the tests compare against (tests/refrecord.py).
 
-Where it comes from:
-  * the build container:  /root/reference (read-only checkout)                      -> `source() == 'checkout'`
-  * the GPU box:          baseline/_ref  (pip install --no-deps --target, git-ignored, travels with gpurun; DESIGN.md §10)
+Where it comes from: the checkout named by $PPQ_REFERENCE_ROOT, else baseline/_ref (`pip install --no-deps --target baseline/_ref`,
+git-ignored; DESIGN.md §10).
 
-Two shims are needed in this image (SURVEY.md §0 fact 6): the stale caffe protobuf module needs the pure-python protobuf
-implementation, and every exporter imports `onnx` (absent) at package import time.  Neither touches the path under test.
+Two shims are needed (SURVEY.md §0 fact 6): the stale caffe protobuf module needs the pure-python protobuf implementation, and every
+exporter imports `onnx` (absent) at package import time.  Neither touches the path under test.
 """
-import importlib.util
 import os
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-_CANDIDATES = [os.environ.get('PPQ_REFERENCE_ROOT', '/root/reference'), os.path.join(ROOT, 'baseline', '_ref')]
-REF_SO = os.path.join(ROOT, 'oracle', '_ref', 'PPQ_Cuda_Impls_ref.so')
+_CANDIDATES = [os.environ.get('PPQ_REFERENCE_ROOT'), os.path.join(ROOT, 'baseline', '_ref')]
 
 
 def root():
@@ -40,16 +38,6 @@ def load():
         sys.path.insert(0, r)
     import ppq
     return ppq
-
-
-def reference_cuda_extension():
-    """The reference's own CUDA extension compiled unmodified for sm_100a (oracle/build_ref.py), or None."""
-    if not os.path.exists(REF_SO):
-        return None
-    spec = importlib.util.spec_from_file_location('PPQ_Cuda_Impls_ref', REF_SO)
-    m = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(m)
-    return m
 
 
 class use_extension:

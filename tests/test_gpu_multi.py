@@ -58,7 +58,7 @@ def _worker(rank, world, port, out_dir):
 
 
 def test_config5_two_ranks_over_nccl_equal_the_single_process_calibration(tmp_path):
-    if torch.cuda.device_count() < 2: pytest.skip('needs 2 GPUs (gpurun --gpus 2)')
+    if torch.cuda.device_count() < 2: pytest.skip('needs 2 GPUs')
     import torch.multiprocessing as mp
     from ppq_b200.calibration import ArenaCalibrator
     world, port = 2, _free_port()
@@ -76,7 +76,7 @@ def test_config5_two_ranks_over_nccl_equal_the_single_process_calibration(tmp_pa
 
 
 def test_one_process_two_devices():
-    if torch.cuda.device_count() < 2: pytest.skip('needs 2 GPUs (gpurun --gpus 2)')
+    if torch.cuda.device_count() < 2: pytest.skip('needs 2 GPUs')
     from ppq_b200.ffi import extension
     ext = extension()
     res = []

@@ -1,19 +1,17 @@
 """GPU parity of the "next" rows (SURVEY.md §8f): Quantile_T / Isotone_T by radix select, LSQ backward, float backward,
-TensorClip, RoundingLoss -- against the reference's own CUDA kernels (oracle/_ref) where present, and against the oracle /
-the torch formulas of the reference's test (tests/test_cuda_kernel.py:66-143) otherwise.
+TensorClip, RoundingLoss -- against the original project's own CUDA kernels (their outputs for these seeded inputs are stored in
+tests/golden/ref_cuda_next_rows.json, see tests/refrecord.py), and against the oracle / the torch formulas of the original's test
+(tests/test_cuda_kernel.py:66-143).
 Element-wise outputs must be bit-identical; scalar fp32 reductions (grad_s, loss) to 1e-4 relative (the reference's own bar is SNR 1e-3)."""
-import importlib.util
-import os
 from math import sqrt
 
 import numpy as np
 import pytest
 import torch
 
-from conftest import ROOT
+import refrecord
 
 pytestmark = pytest.mark.gpu
-REF_SO = os.path.join(ROOT, 'oracle', '_ref', 'PPQ_Cuda_Impls_ref.so')
 
 
 @pytest.fixture(scope='module')
@@ -28,23 +26,21 @@ def ext():
 def ref():
     if not torch.cuda.is_available():
         pytest.skip('no CUDA device')
-    if not os.path.exists(REF_SO):
-        return None
-    spec = importlib.util.spec_from_file_location('PPQ_Cuda_Impls_ref', REF_SO)
-    m = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(m)
-    return m
+    return refrecord.reference_extension()
 
 
-def same_bits(a, b):
-    return torch.equal(a.contiguous().view(torch.int32), b.contiguous().view(torch.int32))
+@pytest.fixture(scope='module')
+def rec(ref):
+    r = refrecord.Record('ref_cuda_next_rows', recording=ref is not None)
+    yield r
+    r.save()
 
 
 def close(a, b, rtol=1e-4, atol=1e-6):
     return torch.allclose(a.double(), b.double(), rtol=rtol, atol=atol)
 
 
-def test_quantile_vs_sort_oracle_and_reference(ext, ref, oracle):
+def test_quantile_vs_sort_oracle_and_reference(ext, ref, rec, oracle):
     g = torch.Generator(device='cuda').manual_seed(0)
     for n in (1, 2, 3, 17, 1000, 4099, 401408, (1 << 21) + 5):
         for kind in ('randn', 'relu', 'negrelu', 'const', 'ints', 'close'):
@@ -66,9 +62,8 @@ def test_quantile_vs_sort_oracle_and_reference(ext, ref, oracle):
                 assert torch.equal(got, want), (n, kind, q, got, want)          # value equality (-0.0 == +0.0)
                 if n <= 4099:
                     assert np.array_equal(got.cpu().numpy(), oracle.quantile_t(x.cpu().numpy(), q)), (n, kind, q)
-                if ref is not None and n > 1:
-                    r = ref.Quantile_T(x, q)
-                    assert torch.equal(got, r) and same_bits(torch.where(got == 0, torch.zeros_like(got), got), torch.where(r == 0, torch.zeros_like(r), r)), (n, kind, q)
+                if n > 1:                                                         # bits with -0.0 read as +0.0
+                    rec.bits(f'Quantile_T n {n} {kind} q {q}', refrecord.plus_zero(got), lambda: refrecord.plus_zero(ref.Quantile_T(x, q)))
     # unaligned view + non-contiguous input
     base = torch.randn(10007, device='cuda', generator=g)
     v = base[1:]
@@ -102,7 +97,7 @@ def test_multi_tensor_quantile_matches_single_launches(ext):
         ext.Multi_Quantile_T(descs, max(sizes), 0.5, torch.zeros(len(xs), 2, device='cuda'), 2, torch.empty(16, dtype=torch.uint8, device='cuda'), 64, None)
 
 
-def test_cold_quantile_with_thresholds_from_a_sample(ext, ref):
+def test_cold_quantile_with_thresholds_from_a_sample(ext, ref, rec):
     """Tensors of >= 8 M elements: a cold Quantile_T draws 16384 samples in its init CTA and speculates on thresholds derived from them (select.cu,
     "self-speculation").  Whatever the sample says, the result must be the exact order statistics: well-behaved data, post-ReLU zeros and clipped
     maxima (the threshold key itself is massively repeated), a constant, few outliers the sample cannot see, structure with the sampling period,
@@ -118,7 +113,7 @@ def test_cold_quantile_with_thresholds_from_a_sample(ext, ref):
         srt = torch.sort(x)[0]
         ia = int(min(max(np.rint(np.float32(n) * np.float32(q)), 0), n - 1)); ib = int(min(max(np.rint(np.float32(n) * (np.float32(1) - np.float32(q))), 0), n - 1))
         assert torch.equal(got, torch.stack([srt[ia], srt[ib]])), (tag, q, got, srt[ia], srt[ib])
-        if ref is not None: assert torch.equal(got, ref.Quantile_T(x, q)), (tag, q)
+        rec.bits(f'cold Quantile_T {tag} q {q}', refrecord.plus_zero(got), lambda: refrecord.plus_zero(ref.Quantile_T(x, q)))
         ext.set_variant('select', 64)                                        # the same call without the sample: the regular two-pass route
         try: assert torch.equal(ext.Quantile_T(x, q), got), (tag, q)
         finally: ext.set_variant('select', 0)
@@ -182,7 +177,7 @@ def test_speculative_quantile_over_consecutive_batches(ext):
         assert bool((gk[:, :, 3] == 0).all())                                   # layout: {threshold, last key, margin, 0} per side
 
 
-def test_isotone_top2_bottom2(ext, ref):
+def test_isotone_top2_bottom2(ext, ref, rec):
     g = torch.Generator(device='cuda').manual_seed(1)
     for n in (1, 2, 5, 1000, 100003):
         x = torch.randn(n, device='cuda', generator=g)
@@ -190,8 +185,8 @@ def test_isotone_top2_bottom2(ext, ref):
         s = torch.sort(x)[0]
         want = torch.stack([s[-1], s[-2], s[0], s[1]]) if n > 1 else torch.stack([s[0]] * 4)
         assert torch.equal(got, want), n
-        if ref is not None and n > 1:
-            assert same_bits(got, ref.Isotone_T(x)), n
+        if n > 1:
+            rec.bits(f'Isotone_T n {n}', got, lambda: ref.Isotone_T(x))
 
 
 def test_percentile_observer_end_to_end(ext):
@@ -227,7 +222,7 @@ def lsq_reference(value, dy, scale, offset, qmin, qmax, c=None):
     return dx, ds
 
 
-def test_lsq_backward_t_and_c(ext, ref):
+def test_lsq_backward_t_and_c(ext, ref, rec):
     g = torch.Generator(device='cuda').manual_seed(3)
     for shape, c in (([1, 1, 1, 1], 1), ([5, 12, 13, 4], 1), ([12, 74, 15, 41], 1), ([501, 7, 73, 1], 0), ([10, 10, 14, 47], 3), ([8192 * 3], 0)):
         for sym in (True, False):
@@ -239,12 +234,11 @@ def test_lsq_backward_t_and_c(ext, ref):
             dx, ds = lsq_reference(t, dy, s, o, 0, 255)
             assert torch.equal(gx, dx), (shape, sym)
             assert close(gs, (ds.double().sum() / sqrt(t.numel() * 255)).float().view(1), rtol=1e-3), (shape, sym)
-            if ref is not None:
-                rx, rs = ref.QuantizeTensor_LT_B(t, s, o, dy, 0, 255, 0)
-                assert same_bits(gx, rx), (shape, sym)
-                # the reference kernel block-reduces inside `if (index < N)` with __syncthreads (linear.cu:252-281): its grad_s is only
-                # well defined when N is a multiple of the 1024-thread block
-                if t.numel() % 1024 == 0: assert close(gs, rs, rtol=1e-3), (shape, sym)
+            key = f'LT_B {shape} sym {sym}'
+            rec.bits(key + ' grad_x', gx, lambda: ref.QuantizeTensor_LT_B(t, s, o, dy, 0, 255, 0)[0])
+            # the reference kernel block-reduces inside `if (index < N)` with __syncthreads (linear.cu:252-281): its grad_s is only
+            # well defined when N is a multiple of the 1024-thread block
+            if t.numel() % 1024 == 0: rec.values(key + ' grad_s', gs, lambda: ref.QuantizeTensor_LT_B(t, s, o, dy, 0, 255, 0)[1], rtol=1e-3, atol=1e-6)
             if len(shape) > 1:
                 C = shape[c]
                 sc = torch.rand(C, device='cuda', generator=g) + 0.01
@@ -254,12 +248,12 @@ def test_lsq_backward_t_and_c(ext, ref):
                 assert torch.equal(gx, dx), (shape, sym, 'C')
                 want = ds.double().transpose(0, c).flatten(1).sum(dim=-1) / sqrt(t.numel() * 255)      # the kernel's factor is rsqrt(N * qmax) (linear.cu:402)
                 assert close(gs, want.float(), rtol=1e-3, atol=1e-5), (shape, sym, 'C')
-                if ref is not None:
-                    rx, rs = ref.QuantizeTensor_LC_B(t, sc, oc, dy, 0, 255, 0, c)
-                    assert same_bits(gx, rx) and close(gs, rs, rtol=1e-3, atol=1e-5), (shape, sym, 'C')
+                key = f'LC_B {shape} axis {c} sym {sym}'
+                rec.bits(key + ' grad_x', gx, lambda: ref.QuantizeTensor_LC_B(t, sc, oc, dy, 0, 255, 0, c)[0])
+                rec.values(key + ' grad_s', gs, lambda: ref.QuantizeTensor_LC_B(t, sc, oc, dy, 0, 255, 0, c)[1], rtol=1e-3, atol=1e-5)
 
 
-def test_float_backward(ext, ref):
+def test_float_backward(ext, ref, rec):
     g = torch.Generator(device='cuda').manual_seed(4)
     x = torch.randn(1024 * 64, device='cuda', generator=g) * 200          # sizes on which the reference kernel's block-wide syncs are safe
     dy = torch.rand(x.shape, device='cuda', generator=g)
@@ -268,18 +262,16 @@ def test_float_backward(ext, ref):
     u = x / s
     sat = (u > 449) | (u < -449)          # the backward kernel quantises with the clip range widened by one (floating.cu:157-158)
     assert torch.equal(gx, torch.where(sat, torch.zeros_like(dy), dy))
-    if ref is not None:
-        rx, rs = ref.QuantizeTensor_FT_B(x, s, o, dy, 4, 3, -448.0, 448.0, 0)
-        assert same_bits(gx, rx) and close(gs, rs, rtol=2e-3)
+    rec.bits('FT_B grad_x', gx, lambda: ref.QuantizeTensor_FT_B(x, s, o, dy, 4, 3, -448.0, 448.0, 0)[0])
+    rec.values('FT_B grad_s', gs, lambda: ref.QuantizeTensor_FT_B(x, s, o, dy, 4, 3, -448.0, 448.0, 0)[1], rtol=2e-3, atol=1e-6)
     xc = x.view(8, 8, 1024)
     sc = 2.0 ** torch.randint(-3, 3, (8,), device='cuda', generator=g).float(); oc = torch.zeros(8, device='cuda')
     gx, gs = ext.QuantizeTensor_FC_B(xc, sc, oc, dy.view(8, 8, 1024), 4, 3, -448.0, 448.0, 0, 1)
-    if ref is not None:
-        rx, rs = ref.QuantizeTensor_FC_B(xc, sc, oc, dy.view(8, 8, 1024), 4, 3, -448.0, 448.0, 0, 1)
-        assert same_bits(gx, rx) and close(gs, rs, rtol=2e-3, atol=1e-5)
+    rec.bits('FC_B grad_x', gx, lambda: ref.QuantizeTensor_FC_B(xc, sc, oc, dy.view(8, 8, 1024), 4, 3, -448.0, 448.0, 0, 1)[0])
+    rec.values('FC_B grad_s', gs, lambda: ref.QuantizeTensor_FC_B(xc, sc, oc, dy.view(8, 8, 1024), 4, 3, -448.0, 448.0, 0, 1)[1], rtol=2e-3, atol=1e-5)
 
 
-def test_tensor_clip_and_rounding_loss(ext, ref):
+def test_tensor_clip_and_rounding_loss(ext, ref, rec):
     g = torch.Generator(device='cuda').manual_seed(5)
     for shape, c in (([7], 0), ([5, 12, 13, 4], 1), ([64, 32, 3, 3], 0), ([3, 1000], 1)):
         v = torch.randn(shape, device='cuda', generator=g)
@@ -302,11 +294,13 @@ def test_tensor_clip_and_rounding_loss(ext, ref):
         clipped = (v > s * (127 - o)) | (v < s * (-128 - o))
         assert close(loss_t, (torch.where(clipped, torch.zeros_like(v), (deq - v).abs()).double().sum() / sqrt(v.numel())).float().view(1), rtol=1e-4)
         assert torch.equal(gt, torch.where(clipped, torch.zeros_like(v), torch.where(v > deq, 1.0, -1.0) * dyy) / torch.sqrt(torch.tensor(float(v.numel()), device='cuda')))
-        if ref is not None:
-            assert same_bits(ext.TensorClip_T(v, r, lim), ref.TensorClip_T(v, r, lim)) and same_bits(ext.TensorClip_C(v, r, limc, c), ref.TensorClip_C(v, r, limc, c))
-            assert close(loss_t, ref.RoundingLoss_LT(v, s, o, -128, 127, 0)) and close(loss_c, ref.RoundingLoss_LC(v, sc, oc, -128, 127, c, 0))
-            assert same_bits(gt, ref.RoundingLoss_LT_B(v, dyy, s, o, -128, 127, 0)), shape
-            assert same_bits(gc, ref.RoundingLoss_LC_B(v, dyy, sc, oc, -128, 127, c, 0)), shape
+        key = f'{shape} axis {c}'
+        rec.bits('TensorClip_T ' + key, ext.TensorClip_T(v, r, lim), lambda: ref.TensorClip_T(v, r, lim))
+        rec.bits('TensorClip_C ' + key, ext.TensorClip_C(v, r, limc, c), lambda: ref.TensorClip_C(v, r, limc, c))
+        rec.values('RoundingLoss_LT ' + key, loss_t, lambda: ref.RoundingLoss_LT(v, s, o, -128, 127, 0), rtol=1e-4, atol=1e-6)
+        rec.values('RoundingLoss_LC ' + key, loss_c, lambda: ref.RoundingLoss_LC(v, sc, oc, -128, 127, c, 0), rtol=1e-4, atol=1e-6)
+        rec.bits('RoundingLoss_LT_B ' + key, gt, lambda: ref.RoundingLoss_LT_B(v, dyy, s, o, -128, 127, 0))
+        rec.bits('RoundingLoss_LC_B ' + key, gc, lambda: ref.RoundingLoss_LC_B(v, dyy, sc, oc, -128, 127, c, 0))
 
 
 def test_culsq_autograd_functions(ext):

@@ -12,7 +12,7 @@ import numpy as np
 import pytest
 import torch
 
-from conftest import ROOT, cases_of, load_golden
+from conftest import ROOT, cases_of, golden_input, load_golden
 
 pytestmark = pytest.mark.gpu
 
@@ -197,7 +197,7 @@ def test_lc_golden_reference_vectors(ext):
     g = load_golden('linear_c.npz')
     for c in cases_of(g):
         k = c['k']
-        x, s, o = dev(g[f'x{k}']), dev(g[f's{k}']), dev(g[f'o{k}'])
+        x, s, o = dev(golden_input(g, c)), dev(g[f's{k}']), dev(g[f'o{k}'])
         y = ext.QuantizeTensor_LC(x, s, o, c['qmin'], c['qmax'], c['axis'], c['mode'])
         assert_bits_equal(y, g[f'y{k}'], f'LC golden case {c}')
         q = ext.QuantizeTensor_toInt(x, s, o, c['qmin'], c['qmax'], c['axis'], c['mode'], 32)

@@ -8,9 +8,9 @@ import json
 import os
 
 import numpy as np
-import pytest
 
-from conftest import GOLDEN, cases_of, load_golden, seeded_batches
+import refrecord
+from conftest import GOLDEN, cases_of, golden_input, load_golden, seeded_batches
 
 
 def bits(a):
@@ -47,7 +47,7 @@ def test_linear_c_matches_reference_cpu_path(oracle):
     g = load_golden('linear_c.npz')
     for c in cases_of(g):
         k = c['k']
-        x, y_ref, q_ref, s, o = g[f'x{k}'], g[f'y{k}'], g[f'q{k}'], g[f's{k}'], g[f'o{k}']
+        x, y_ref, q_ref, s, o = golden_input(g, c), g[f'y{k}'], g[f'q{k}'], g[f's{k}'], g[f'o{k}']
         y, q = oracle.linear_quant_c(x, s, o, c['axis'], c['qmin'], c['qmax'], c['mode'], return_int=True)
         assert np.array_equal(q, q_ref), c
         assert np.array_equal(bits(y), bits(y_ref)), c
@@ -176,20 +176,23 @@ def test_compute_mse_loss_vs_reference_cpp(oracle):
 
 
 def test_compute_mse_loss_vs_live_reference_build(oracle):
-    """When oracle/_ref/hist_mse_ref.so (the reference's hist_mse.cc compiled in place) is present, fuzz against it."""
+    """200 seeded cases against the reference's hist_mse.cc compiled in place (oracle/_ref/hist_mse_ref.so); its results are stored in
+    tests/golden/ref_hist_mse.json (tests/refrecord.py: recorded with PPQ_RECORD_GOLDEN set and oracle/_ref built)."""
     import ctypes
-    so = os.path.join(os.path.dirname(GOLDEN), '..', 'oracle', '_ref', 'hist_mse_ref.so')
-    if not os.path.exists(so):
-        pytest.skip('oracle/_ref not built on this machine')
-    lib = ctypes.CDLL(so)
-    lib.ref_compute_mse_loss.restype = ctypes.c_float
-    lib.ref_compute_mse_loss.argtypes = [ctypes.c_void_p, ctypes.c_int64, ctypes.c_int, ctypes.c_int, ctypes.c_int]
+    recording = refrecord.record_dir() is not None
+    if recording:
+        lib = ctypes.CDLL(os.path.join(os.path.dirname(GOLDEN), '..', 'oracle', '_ref', 'hist_mse_ref.so'))
+        lib.ref_compute_mse_loss.restype = ctypes.c_float
+        lib.ref_compute_mse_loss.argtypes = [ctypes.c_void_p, ctypes.c_int64, ctypes.c_int, ctypes.c_int, ctypes.c_int]
+    rec = refrecord.Record('ref_hist_mse', recording=recording)
     r = np.random.RandomState(99)
-    for _ in range(200):
+    for i in range(200):
         nb = int(r.choice([16, 100, 2048]))
         h = r.randint(0, 5000, size=nb).astype(np.int64)
         step = int(r.randint(1, 9)); start = int(r.randint(0, nb // 2)); end = start + int(r.randint(1, 300)) * step
-        assert np.float32(oracle.compute_mse_loss(h, start, step, end)) == np.float32(lib.ref_compute_mse_loss(h.ctypes.data, nb, start, step, end))
+        rec.values(f'{i} bins {nb} start {start} step {step} end {end}', np.float32(oracle.compute_mse_loss(h, start, step, end)),
+                   lambda: np.float32(lib.ref_compute_mse_loss(h.ctypes.data, nb, start, step, end)), rtol=0)
+    rec.save()
 
 
 def test_fp8_restatement_sanity(oracle):
