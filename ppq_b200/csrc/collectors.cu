@@ -8,7 +8,7 @@
 //   ppq_b200_multi_*                one launch over a table of tensors (the calibration arena path, DESIGN.md)
 //
 // All of them read each element exactly once (4 B/element algorithmic traffic) with 128-bit streaming loads, four per
-// thread in flight.  Histograms are privatised per CTA in shared memory (bins x int32, 16 KB for the KL observer's 4096
+// thread in flight (the multi-tensor min/max and histogram: 256-bit loads, see stream_v8).  Histograms are privatised per CTA in shared memory (bins x int32, 16 KB for the KL observer's 4096
 // bins) and counted with an unconditional red.shared.add into `bins + 1` slots (the extra one is a trash slot for dropped
 // samples; ptxas emits ATOMS.POPC.INC, which aggregates same-address lanes in hardware, so the post-ReLU pile-up in bin 0 is
 // not a hot spot); only non-empty bins are flushed to the caller's global histogram with red.global.add.
@@ -379,6 +379,138 @@ histogram_c_kernel(const float *__restrict__ x, int64_t rows, int64_t epc, int C
     }
 }
 
+// ---- multi-tensor streaming collectors ---------------------------------------------------------------------------------
+// The launch reads the concatenation of all tensors once.  Every CTA owns one contiguous span of equal length of that
+// concatenation (no empty work items however ragged the table is) and walks the tensors overlapping it; a CTA's statistics
+// for one tensor are published once.  Loads are 256-bit (LDG.E.256 on sm_100a), U per thread in flight, lane-interleaved
+// inside warp-contiguous segments; the head up to the first 32-byte boundary and the ragged tail go through scalar loads,
+// so any 4-byte aligned base is on the vector path.
+
+struct float8v { float4 a, b; };
+__device__ __forceinline__ float8v ld_stream8(const float *p) {
+    float8v v;
+    asm volatile("ld.global.nc.L1::no_allocate.L2::evict_first.L2::256B.v8.f32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
+                 : "=f"(v.a.x), "=f"(v.a.y), "=f"(v.a.z), "=f"(v.a.w), "=f"(v.b.x), "=f"(v.b.y), "=f"(v.b.z), "=f"(v.b.w) : "l"(p));
+    return v;
+}
+
+// Elements [0, n) of x, split over `nthreads` threads of the calling CTA: f4(float4) for vector data, f1(float) for the
+// head and tail elements.
+template <int U, class F4, class F1>
+__device__ __forceinline__ void stream_v8(const float *__restrict__ x, int64_t n, int tid, int nthreads, F4 &&f4, F1 &&f1) {
+    const int64_t to_boundary = (int64_t)(((32u - ((uint32_t)reinterpret_cast<uintptr_t>(x) & 31u)) & 31u) >> 2);
+    const int head = (int)(to_boundary < n ? to_boundary : n);
+    if (tid < head) f1(ld_stream1(x + tid));
+    x += head; n -= head;
+    const float *const end = x + (n & ~(int64_t)7);                    // end of the vector part
+    constexpr int kSeg = 32 * 8 * U;                                   // floats per warp segment
+    const int64_t step = (int64_t)(nthreads >> 5) * kSeg;
+    for (const float *p = x + (int64_t)(tid >> 5) * kSeg + (tid & 31) * 8; p < end; p += step) {
+        float8v v[U];
+#pragma unroll
+        for (int j = 0; j < U; j++) if (p + j * 256 < end) v[j] = ld_stream8(p + j * 256);
+#pragma unroll
+        for (int j = 0; j < U; j++) if (p + j * 256 < end) { f4(v[j].a); f4(v[j].b); }
+    }
+    const float *t = end + tid;
+    if (t < x + n) f1(ld_stream1(t));
+}
+
+// prefix[t] = elements of tensors 0 .. t-1 (prefix[count] = total), built in shared memory by the whole CTA: one parallel
+// round of descriptor loads, then a chunked warp scan.
+__device__ __forceinline__ int64_t build_prefix(const ppq_b200_tensor_desc *__restrict__ descs, int count, int64_t *prefix) {
+    for (int i = threadIdx.x; i < count; i += blockDim.x) { const int64_t n = descs[i].n; prefix[i + 1] = n > 0 ? n : 0; }
+    if (threadIdx.x == 0) prefix[0] = 0;
+    __syncthreads();
+    if (threadIdx.x < 32) {
+        const int lane = threadIdx.x;
+        int64_t carry = 0;
+        for (int b = 1; b <= count; b += 32) {
+            const int i = b + lane;
+            int64_t v = i <= count ? prefix[i] : 0;
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) { const int64_t w = __shfl_up_sync(0xffffffffu, v, o); if (lane >= o) v += w; }
+            v += carry;
+            if (i <= count) prefix[i] = v;
+            carry = __shfl_sync(0xffffffffu, v, 31);
+        }
+    }
+    __syncthreads();
+    return prefix[count];
+}
+
+// This CTA's span [s0, s1) of the concatenation and the first tensor overlapping it; false when the span is empty.
+__device__ __forceinline__ bool cta_span(const int64_t *prefix, int count, int64_t total, int64_t &s0, int64_t &s1, int &t) {
+    const int64_t span = (total + gridDim.x - 1) / gridDim.x;
+    s0 = (int64_t)blockIdx.x * span;
+    s1 = min(s0 + span, total);
+    if (s0 >= total) return false;
+    int lo = 0, hi = count - 1;                                        // last t with prefix[t] <= s0
+    while (lo < hi) { const int mid = (lo + hi + 1) >> 1; if (prefix[mid] <= s0) lo = mid; else hi = mid - 1; }
+    t = lo;
+    return true;
+}
+
+// min/max: each warp folds its share of a (CTA, tensor) piece in registers and publishes it with two atomics, no CTA barrier.
+template <int TPB, int MINB, int U>
+__global__ void __launch_bounds__(TPB, MINB)
+multi_minmax_stream_kernel(const ppq_b200_tensor_desc *__restrict__ descs, int count, float *__restrict__ arena) {
+    extern __shared__ int64_t prefix[];
+    const int64_t total = build_prefix(descs, count, prefix);
+    int64_t s0, s1; int t;
+    if (!cta_span(prefix, count, total, s0, s1, t)) return;
+    for (; t < count && prefix[t] < s1; t++) {
+        const ppq_b200_tensor_desc d = descs[t];
+        const int64_t a = max(s0 - prefix[t], (int64_t)0), b = min(s1 - prefix[t], d.n);
+        if (b <= a) continue;                                          // uniform per CTA
+        MinMax mm;
+        stream_v8<U>(d.x + a, b - a, threadIdx.x, TPB, [&](const float4 &v) { mm.add4(v); }, [&](float v) { mm.add(v); });
+        mm.warp_reduce();
+        const bool empty = mm.lo == __int_as_float(0x7F800000) && mm.hi == __int_as_float(0xFF800000);   // warp saw no element
+        if ((threadIdx.x & 31) == 0 && !empty) mm.publish(arena + 2 * (int64_t)d.slot, arena + 2 * (int64_t)d.slot + 1);
+    }
+}
+
+// SymBin's slot with a full-rate floor: for 0 <= u < 2^23, u + 2^23 rounded down is 2^23 + floor(u), whose bit pattern is
+// 0x4B000000 + floor(u).  Clamping the quotient to [0, cap] before the floor gives min(floor(q), cap) as SymBin does
+// (cap = bins: the trash slot, or bins - 1), and fmaxf sends a NaN quotient to slot 0 like F2I.  The slot's byte address in
+// the shared histogram is folded into one integer multiply-add of the float's bits.
+struct SymSlot {
+    ExactDiv d; float cap; uint32_t base;
+    __device__ __forceinline__ SymSlot(float hist_scale, int bins, bool clip, const int *sh)
+        : cap((float)(clip ? bins : bins - 1)), base((uint32_t)__cvta_generic_to_shared(sh) - 0x4B000000u * 4u) { d.init(hist_scale); }
+    __device__ __forceinline__ uint32_t addr(float q) const {
+        return base + __float_as_uint(__fadd_rd(fminf(fmaxf(q, 0.f), cap), 8388608.f)) * 4u;
+    }
+    __device__ __forceinline__ static void count(uint32_t a) { asm volatile("red.shared.add.u32 [%0], 1;" ::"r"(a) : "memory"); }
+    __device__ __forceinline__ void add(float v) const { count(addr(d.div(fabsf(v)))); }
+    __device__ __forceinline__ void add4(const float4 &v) const {
+        const float4 q = d.div4(make_float4(fabsf(v.x), fabsf(v.y), fabsf(v.z), fabsf(v.w)));
+        count(addr(q.x)); count(addr(q.y)); count(addr(q.z)); count(addr(q.w));
+    }
+};
+
+template <int TPB, int MINB, int U>
+__global__ void __launch_bounds__(TPB, MINB)
+multi_histogram_stream_kernel(const ppq_b200_tensor_desc *__restrict__ descs, int count, const float *__restrict__ hist_scale_arena,
+                              int clip, int bins, int32_t *__restrict__ hist_arena) {
+    extern __shared__ int sh[];
+    int64_t *prefix = reinterpret_cast<int64_t *>(sh + ((bins + 1 + 1) & ~1));   // [count + 1], 8-byte aligned
+    const int64_t total = build_prefix(descs, count, prefix);
+    int64_t s0, s1; int t;
+    if (!cta_span(prefix, count, total, s0, s1, t)) return;
+    for (; t < count && prefix[t] < s1; t++) {
+        const ppq_b200_tensor_desc d = descs[t];
+        const int64_t a = max(s0 - prefix[t], (int64_t)0), b = min(s1 - prefix[t], d.n);
+        if (b <= a) continue;                                          // uniform per CTA
+        int32_t *gh = hist_arena + (int64_t)d.slot * bins;
+        hist_zero<0>(sh, bins);
+        const SymSlot bin(__ldg(hist_scale_arena + d.slot), bins, clip != 0, sh);
+        stream_v8<U>(d.x + a, b - a, threadIdx.x, TPB, [&](const float4 &v) { bin.add4(v); }, [&](float v) { bin.add(v); });
+        hist_flush<0>(sh, bins, gh);
+    }
+}
+
 // ---- launch helpers -------------------------------------------------------------------------------------------------------
 constexpr int kMaxSmemBins = 12287;            // (bins + 1) int32 slots within the default 48 KB of dynamic shared memory
 
@@ -414,6 +546,29 @@ static int launch_hist(const float *x, int64_t n, const BinParams &bin, int64_t 
     // default: two 1024-thread CTAs per SM (32 registers per thread), 2 loads in flight per thread
     default: histogram_kernel<0, Bin, 2, kHistThreads, 2><<<grid * 2 > sm_count() * 2 ? sm_count() * 2 : grid * 2, kHistThreads, smem, st>>>(x, n, bin, hist); break;
     }
+    return (int)cudaGetLastError();
+}
+
+// Multi-tensor stream launches: one full wave of MINB CTAs per SM, each owning an equal span of the concatenation.  Both run 2 x 512
+// threads per SM with 4 x 256-bit loads per thread in flight (128 KB per SM); measured on B200 against 512 x 4 (U 2), 1024 x 1 and,
+// for the histogram, 1024 x 1 (U 2 / U 4) and 512 x 3 (U 2): profiles/r03_ab_explore.txt.
+constexpr size_t kMaxPrefixSmem = 200 * 1024;  // descriptor prefix of the min/max launch: up to ~25 k tensors
+
+template <int TPB, int MINB, int U>
+static int launch_multi_minmax(const ppq_b200_tensor_desc *descs, int count, size_t smem, float *arena, cudaStream_t st) {
+    auto k = multi_minmax_stream_kernel<TPB, MINB, U>;
+    if (smem > 48 * 1024) {
+        const cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return (int)e;
+    }
+    k<<<sm_count() * MINB, TPB, smem, st>>>(descs, count, arena);
+    return (int)cudaGetLastError();
+}
+
+template <int TPB, int MINB, int U>
+static int launch_multi_hist(const ppq_b200_tensor_desc *descs, int count, size_t smem, const float *hist_scale_arena, int clip,
+                             int bins, int32_t *hist_arena, cudaStream_t st) {
+    multi_histogram_stream_kernel<TPB, MINB, U><<<sm_count() * MINB, TPB, smem, st>>>(descs, count, hist_scale_arena, clip, bins, hist_arena);
     return (int)cudaGetLastError();
 }
 
@@ -485,6 +640,11 @@ int ppq_b200_histogram_c(const float *x, int64_t n, int64_t epc, int C, float hi
 
 int ppq_b200_multi_minmax_t(const ppq_b200_tensor_desc *descs, int count, int64_t max_n, float *minmax_arena, void *stream) {
     if (count <= 0 || max_n <= 0 || !descs || !minmax_arena) return (int)cudaErrorInvalidValue;
+    if (variant_of(kVarMinMax) != 1) {          // 1: the replaced per-chunk kernel below (A/B only)
+        const size_t smem = (size_t)(count + 1) * sizeof(int64_t);
+        if (smem > kMaxPrefixSmem) return (int)cudaErrorInvalidValue;
+        return launch_multi_minmax<512, 2, 4>(descs, count, smem, minmax_arena, (cudaStream_t)stream);
+    }
     const int64_t chunk = 65536;
     const int64_t cpt = (max_n + chunk - 1) / chunk;
     if (cpt > 0x7fffffffLL) return (int)cudaErrorInvalidValue;
@@ -499,6 +659,9 @@ int ppq_b200_multi_histogram_t(const ppq_b200_tensor_desc *descs, int count, int
     if (count <= 0 || max_n <= 0 || !descs || !hist_scale_arena || !hist_arena || bins <= 0 || bins > kMaxSmemBins) return (int)cudaErrorInvalidValue;
     const size_t smem = (size_t)((bins + 2) & ~1) * sizeof(int) + (size_t)(count + 1) * sizeof(int64_t);
     if (smem > 48 * 1024) return (int)cudaErrorInvalidValue;
+    if (variant_of(kVarMultiHist) != 1) {       // 1: the replaced fixed-span kernel below (A/B only)
+        return launch_multi_hist<512, 2, 4>(descs, count, smem, hist_scale_arena, clip_outliers, (int)bins, hist_arena, (cudaStream_t)stream);
+    }
     // grid: one CTA per SM, fewer when the whole job is small (each CTA should own >= 64 Ki elements before paying for a flush)
     int64_t g = ((int64_t)count * max_n + 65535) / 65536;
     if (g > sm_count()) g = sm_count();

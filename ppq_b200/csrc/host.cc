@@ -19,6 +19,7 @@ static int key_of(const char *name) {
     if (!strcmp(name, "linear_quant_c")) return kVarChannel;
     if (!strcmp(name, "kl_search")) return kVarKlSearch;
     if (!strcmp(name, "select")) return kVarSelect;
+    if (!strcmp(name, "multi_histogram")) return kVarMultiHist;
     return -1;
 }
 }  // namespace ppqb
